@@ -17,6 +17,8 @@ One *step* = one such batch through b200_search_batch (mode 2).  `--mode keyword
             bounded sample of the same queries, fixed thread count, with the latency distribution and a searchCutoffMs-clamped figure
   parity    ALL queries of one timed batch against the oracle: docids, ScoreDetails rank tuples, candidate counts (keyword,
             Detailed) and the merged hybrid hits (docids, scores within 1e-4 relative on the vector similarity)
+  --dump-outputs DIR   the search result of the last timed step as DIR/<array>.npy; the same arguments give the same inputs, so two
+            builds can be compared output for output
 
 Multi-GPU (torchrun): the path shards by query — every rank holds a replica and serves its own batches; no data-path collective
 (DESIGN.md §5); value = all ranks' queries / max-over-ranks time.
@@ -370,6 +372,7 @@ def main():
     ap.add_argument("--parity", type=int, default=0, help="queries of the parity check (0 = the whole batch)")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary vector-stage measurements")
     ap.add_argument("--shard-rows", type=int, default=12_500_000, help="embedding rows per GPU of the corpus-sharded stage (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the search result of the last timed step as DIR/<array>.npy (rank 0)")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -542,9 +545,32 @@ def main():
         out["vector_stage_sharded"] = sharded_vector_stage(args, ix, rank, world, local_rank)
     if not args.no_extras and world == 1:
         extras(args, ix, img, emb, batches, out, peaks)
+    if args.dump_outputs:  # res: the last step of the e2e pass, which runs as production does
+        dump_outputs(res, args.dump_outputs)
     print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+RESULT_ARRAYS = ("documents_ids", "n_hits", "n_scores", "score_kind", "score_rank", "score_max", "score_sim", "n_candidates",
+                 "semantic_hit_count", "status", "degraded", "used_negative_operator")
+DUMP_LIMIT_BYTES = 60 << 20  # array data; with the .npy headers and query_index.npy the files stay below 64 MB
+
+
+def dump_outputs(res, out_dir):
+    """The arrays of a SearchResult as out_dir/<name>.npy, so that two builds can be compared output for output: score_sim stays
+    float32, the integer arrays become float64 (exact: every value is below 2**53).  A batch whose arrays exceed 64 MB is cut to a
+    seeded sample of its queries, whose row numbers go to query_index.npy."""
+    n = len(res.n_hits)
+    per_query = sum((4 if name == "score_sim" else 8) * getattr(res, name)[:1].size for name in RESULT_ARRAYS)
+    keep = min(n, DUMP_LIMIT_BYTES // per_query)
+    rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name in RESULT_ARRAYS:
+        a = getattr(res, name)[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+    if keep < n:
+        np.save(os.path.join(out_dir, "query_index.npy"), rows.astype(np.float64))
 
 
 def extras(args, ix, img, emb, batches, out, peaks):

@@ -187,9 +187,11 @@ class CachedImage:
 
 def synthetic_image(n_docs, vocab, seed=0xB200, n_fields=1, cache_min_docs=2_000_000, log=None):
     """The synthetic corpus of SURVEY §8(d), built (multi-threaded) or restored from B200_CORPUS_CACHE (default
-    /tmp/b200_corpus_cache).  Only corpora of at least cache_min_docs documents are cached; concurrent processes (the ranks of a
-    torchrun launch, the two arms of the bench) build once: the first takes a lock directory, the others wait for its `done` file."""
+    b200_corpus_cache_<uid> in the temporary directory: users sharing a host do not share it).  Only corpora of at least
+    cache_min_docs documents are cached; concurrent processes (the ranks of a torchrun launch, the two arms of the bench) build once:
+    the first takes a lock directory, the others wait for its `done` file.  Without a writable cache directory the corpus is built."""
     import json
+    import tempfile
     import time
 
     def build():
@@ -199,16 +201,18 @@ def synthetic_image(n_docs, vocab, seed=0xB200, n_fields=1, cache_min_docs=2_000
 
     if n_docs < cache_min_docs or os.environ.get("B200_CORPUS_CACHE") == "off":
         return build()
-    root = os.environ.get("B200_CORPUS_CACHE", "/tmp/b200_corpus_cache")
+    root = os.environ.get("B200_CORPUS_CACHE", os.path.join(tempfile.gettempdir(), f"b200_corpus_cache_{os.getuid()}"))
     path = os.path.join(root, f"syn_v3_{n_docs}_{vocab}_{seed:x}_{n_fields}")
     done = os.path.join(path, "done")
-    os.makedirs(root, exist_ok=True)
     if not os.path.exists(done):
         try:
+            os.makedirs(root, exist_ok=True)
             os.mkdir(path)
             owner = True
         except FileExistsError:
             owner = False
+        except OSError:
+            return build()
         if not owner:
             t0 = time.time()
             while not os.path.exists(done) and time.time() - t0 < 1800:
