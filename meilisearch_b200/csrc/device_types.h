@@ -26,6 +26,19 @@ struct LevRec {
     uint32_t pad;
     unsigned long long codes;   // 2 bits per lane: 0 none, 1 same-first d=1, 2 same-first d=2, 3 different-first (d=1)
 };
+// Pruned derivation schedule (built by Engine::derive_batch): a term is only swept over the dictionary words whose first two
+// bytes can pass the first-letter rule.  Those words form groups, each a union of id ranges of the sorted dictionary:
+//   LEV_GROUP_F  (c): words with w[0] == c
+//   LEV_GROUP_S  (c): words with w[1] == c (a one-byte word counts as w[1] == 0), minus those with w[0] in {q[0], q[1]} of the term
+//   LEV_GROUP_ALL   : every word
+constexpr uint8_t LEV_GROUP_F = 0, LEV_GROUP_S = 1, LEV_GROUP_ALL = 2;
+struct LevChunk {     // up to LEV_TERMS_PER_CTA terms of one group
+    uint32_t first;   // into the term index list
+    uint8_t n, kind, c, pad;
+};
+struct LevItem {      // one CTA: one chunk against one 256-word tile that overlaps the chunk's group
+    uint32_t tile, chunk;
+};
 
 // ---- rule activations ----
 constexpr uint32_t MAX_COSTS = 128;

@@ -430,6 +430,7 @@ struct Engine {
     DevBuf<LevTerm> d_lev_terms;
     DevBuf<LevRec> d_lev_recs;
     DevBuf<uint32_t> d_lev_u32;  // rec_count | one_out | n_one | two_out | n_two | status
+    DevBuf<uint32_t> d_lev_sched;  // derivation schedule: LevItem[] | LevChunk[] | term indices
     // vector buffers
     DevBuf<float> d_vq, d_vdist, d_vsel_dist;
     DevBuf<uint32_t> d_vsel_ids, d_vsel_n;

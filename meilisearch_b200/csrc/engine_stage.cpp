@@ -98,6 +98,7 @@ Engine::~Engine() {
     d_lev_terms.release();
     d_lev_recs.release();
     d_lev_u32.release();
+    d_lev_sched.release();
     d_vq.release();
     d_vdist.release();
     d_vsel_dist.release();
@@ -255,6 +256,90 @@ int Engine::stage_embeddings(const float *vectors, const uint16_t *half_rows, ui
     return B200_OK;
 }
 
+// The derivation schedule: which (chunk of terms, 256-word tile) pairs lev_match_kernel visits, one CTA each.
+//
+// Why it is exact.  The kernel's filter lets a (term, word) pair through only when
+//   w[0] == q[0] (budget k_same), or
+//   w[0] != q[0], k_diff >= 0 and (m < 2 or w[1] == q[1] or w[1] == q[0] or w[0] == q[1]),
+// and it rejects every word of a term with k_same < 0 (its first test, popcount > k_same, always holds).  For every term those
+// words are the disjoint union of its groups (device_types.h):
+//   k_same < 0                      none
+//   k_diff < 0                      F(q0)
+//   k_diff >= 0, m < 2              ALL
+//   k_diff >= 0, m >= 2             F(q0), S(q0), and when q1 != q0 also F(q1), S(q1)
+// since F(q1) holds the words with w[0] == q1 != q0, and S(q0) ∪ S(q1) those with w[0] not in {q0, q1} and w[1] in {q0, q1}.
+// A group's tiles cover all of its words, and inside an item the kernel tests a pair only when the word lies in the item's group
+// for that term.  So every pair that a full (tile x term) sweep could pass through the first-byte rule is tested exactly once,
+// by the same filter and DP, and no other pair is.  The records of one 32-word group that two items produce hold disjoint words;
+// lev_finalize_kernel ORs them after sorting by word id, so it replays the 150 / 50 caps over the same codes in the same word-id
+// order and keeps the same words.
+namespace {
+struct LevSchedule {
+    std::vector<LevItem> items;
+    std::vector<LevChunk> chunks;
+    std::vector<uint32_t> term_idx;  // the members of every group, group by group
+    uint64_t bytes = 0;              // dictionary bytes + offsets of the tiles the items stage
+};
+void build_lev_schedule(const HostIndex &ix, const std::vector<LevTerm> &terms, LevSchedule &s) {
+    constexpr uint32_t G_S = 256, G_ALL = 512, N_GROUPS = 513;  // group ids: F(c) = c, S(c) = 256 + c, ALL = 512
+    auto groups_of = [](const LevTerm &t, auto &&add) {
+        if (t.k_same < 0) return;
+        const uint8_t q0 = t.q[0], q1 = t.q[1];
+        if (t.k_diff < 0) {
+            add(q0);
+        } else if (t.len < 2) {
+            add(G_ALL);
+        } else {
+            add(q0);
+            add(G_S + q0);
+            if (q1 != q0) {
+                add(q1);
+                add(G_S + q1);
+            }
+        }
+    };
+    std::vector<uint32_t> first(N_GROUPS + 1, 0);
+    for (const LevTerm &t : terms) groups_of(t, [&](uint32_t g) { first[g + 1]++; });
+    for (uint32_t g = 0; g < N_GROUPS; g++) first[g + 1] += first[g];
+    s.term_idx.resize(first[N_GROUPS]);
+    std::vector<uint32_t> fill(first.begin(), first.end() - 1);
+    for (uint32_t i = 0; i < (uint32_t)terms.size(); i++) groups_of(terms[i], [&](uint32_t g) { s.term_idx[fill[g]++] = i; });
+
+    const uint32_t n_words = (uint32_t)ix.n_words;
+    const std::vector<uint32_t> &start = ix.dict_pair_start;
+    std::vector<uint32_t> tiles;
+    auto add_words = [&](uint32_t lo, uint32_t hi) {  // the tiles of words [lo, hi); ranges come in increasing order
+        if (lo >= hi) return;
+        uint32_t t = lo / 256;
+        if (!tiles.empty() && tiles.back() >= t) t = tiles.back() + 1;
+        for (; t <= (hi - 1) / 256; t++) tiles.push_back(t);
+    };
+    for (uint32_t g = 0; g < N_GROUPS; g++) {
+        if (first[g] == first[g + 1]) continue;
+        tiles.clear();
+        if (g < G_S) {
+            add_words(start[g << 8], start[(g + 1) << 8]);
+        } else if (g < G_ALL) {
+            for (uint32_t b0 = 0; b0 < 256; b0++) add_words(start[b0 << 8 | (g - G_S)], start[(b0 << 8 | (g - G_S)) + 1]);
+        } else {
+            add_words(0, n_words);
+        }
+        uint64_t tile_bytes = 0;
+        for (uint32_t t : tiles) {
+            const uint32_t w0 = t * 256, w1 = std::min(n_words, w0 + 256);
+            tile_bytes += ix.dict_off[w1] - ix.dict_off[w0] + 4ull * (w1 - w0);
+        }
+        const uint8_t kind = g < G_S ? LEV_GROUP_F : (g < G_ALL ? LEV_GROUP_S : LEV_GROUP_ALL);
+        for (uint32_t c0 = first[g]; c0 < first[g + 1]; c0 += LEV_TERMS_PER_CTA) {
+            const uint32_t chunk = (uint32_t)s.chunks.size();
+            s.chunks.push_back(LevChunk{c0, (uint8_t)std::min<uint32_t>(LEV_TERMS_PER_CTA, first[g + 1] - c0), kind, (uint8_t)(g & 255), 0});
+            for (uint32_t t : tiles) s.items.push_back(LevItem{t, chunk});
+            s.bytes += tile_bytes;
+        }
+    }
+}
+}  // namespace
+
 int Engine::derive_batch(uint32_t n, const char *words, const uint32_t *off, const uint8_t *max_typo, const uint8_t *is_prefix,
                          uint32_t *one_out, uint32_t *n_one, uint32_t *two_out, uint32_t *n_two) {
     if (!staged) return fail(B200_ERR_STATE, "derive before b200_stage_finish");
@@ -280,18 +365,28 @@ int Engine::derive_batch(uint32_t n, const char *words, const uint32_t *off, con
     uint32_t *rec_count = d_lev_u32.p, *d_one = rec_count + n, *d_n_one = d_one + (size_t)n * 150, *d_two = d_n_one + n,
              *d_n_two = d_two + (size_t)n * 50;
     int32_t *d_status = reinterpret_cast<int32_t *>(d_n_two + n);
+    LevSchedule sched;
+    build_lev_schedule(hix, terms, sched);
+    static_assert(sizeof(LevItem) % 4 == 0 && sizeof(LevChunk) % 4 == 0, "schedule layout");
+    const size_t items_u32 = sched.items.size() * sizeof(LevItem) / 4, chunks_u32 = sched.chunks.size() * sizeof(LevChunk) / 4;
+    CU(d_lev_sched.reserve(items_u32 + chunks_u32 + sched.term_idx.size()), "alloc lev schedule");
+    const LevItem *d_items = reinterpret_cast<const LevItem *>(d_lev_sched.p);
+    const LevChunk *d_chunks = reinterpret_cast<const LevChunk *>(d_lev_sched.p + items_u32);
+    const uint32_t *d_term_idx = d_lev_sched.p + items_u32 + chunks_u32;
     CU(cudaMemcpyAsync(d_lev_terms.p, terms.data(), n * sizeof(LevTerm), cudaMemcpyHostToDevice, stream), "H2D lev terms");
-    stats.h2d_bytes += n * sizeof(LevTerm);
+    CU(cudaMemcpyAsync((void *)d_items, sched.items.data(), items_u32 * 4, cudaMemcpyHostToDevice, stream), "H2D lev schedule");
+    CU(cudaMemcpyAsync((void *)d_chunks, sched.chunks.data(), chunks_u32 * 4, cudaMemcpyHostToDevice, stream), "H2D lev schedule");
+    CU(cudaMemcpyAsync((void *)d_term_idx, sched.term_idx.data(), sched.term_idx.size() * 4, cudaMemcpyHostToDevice, stream), "H2D lev schedule");
+    stats.h2d_bytes += n * sizeof(LevTerm) + (items_u32 + chunks_u32 + sched.term_idx.size()) * 4;
     stats.d2h_bytes += (size_t)n * (150 + 50 + 3) * 4;
     size_t m0 = mark();
-    CU(launch_lev(stream, dix.dict_bytes, dix.dict_off, (uint32_t)hix.n_words, d_lev_terms.p, n, d_lev_recs.p, rec_count, d_one, d_n_one, d_two,
-                  d_n_two, d_status),
+    CU(launch_lev(stream, dix.dict_bytes, dix.dict_off, (uint32_t)hix.n_words, d_lev_terms.p, n, d_term_idx, d_chunks, d_items,
+                  (uint32_t)sched.items.size(), d_lev_recs.p, rec_count, d_one, d_n_one, d_two, d_n_two, d_status),
        "lev kernels");
     size_t m1 = mark();
-    uint64_t lev_bytes = (uint64_t)((n + LEV_TERMS_PER_CTA - 1) / LEV_TERMS_PER_CTA) * (hix.dict_bytes.size() + 4 * hix.n_words);
-    time_kernel(B200_K_LEV, m0, m1, lev_bytes);
+    time_kernel(B200_K_LEV, m0, m1, sched.bytes);
     stats.kernel_launches += 1;
-    stats.dictionary_bytes += lev_bytes;
+    stats.dictionary_bytes += sched.bytes;
     std::vector<int32_t> status(n);
     CU(cudaMemcpyAsync(one_out, d_one, (size_t)n * 150 * 4, cudaMemcpyDeviceToHost, stream), "D2H");
     CU(cudaMemcpyAsync(n_one, d_n_one, (size_t)n * 4, cudaMemcpyDeviceToHost, stream), "D2H");

@@ -141,6 +141,16 @@ void build_host_index(const std::vector<uint8_t> &dict_bytes, const std::vector<
     ix.dict_off = dict_off;
     ix.n_words = dict_off.empty() ? 0 : dict_off.size() - 1;
     if (ix.n_words >= (1u << 21)) throw std::runtime_error("stage: dictionary larger than 2^21 words (packed pair keys)");
+    // first word id per leading byte pair (the term derivation schedule's word ranges)
+    ix.dict_pair_start.assign(65537, 0);
+    for (uint64_t i = 0, prev = 0; i < ix.n_words; i++) {
+        const size_t n = ix.word_len(i);
+        const uint32_t key = n == 0 ? 0u : ((uint32_t)ix.word_ptr(i)[0] << 8) | (n > 1 ? ix.word_ptr(i)[1] : 0u);
+        if (key < prev) throw std::runtime_error("stage: dictionary words are not in bytewise order");
+        prev = key;
+        ix.dict_pair_start[key + 1]++;
+    }
+    for (uint32_t k = 0; k < 65536; k++) ix.dict_pair_start[k + 1] += ix.dict_pair_start[k];
     // universe
     std::vector<uint32_t> docs;
     cbo_decode_append(docids_cbo.data(), docids_cbo.size(), docs);

@@ -54,6 +54,10 @@ struct HostIndex {
     std::vector<uint8_t> dict_bytes;
     std::vector<uint64_t> dict_off;
     uint64_t n_words = 0;
+    // dict_pair_start[b0 << 8 | b1] = first word id whose first two bytes are >= (b0, b1), 65537 entries (the last = n_words).
+    // The dictionary is sorted, so the words with first byte c are [start[c << 8], start[(c + 1) << 8]) and those with first
+    // bytes (b0, c) are [start[b0 << 8 | c], start[(b0 << 8 | c) + 1]).  A one-byte word counts as second byte 0.
+    std::vector<uint32_t> dict_pair_start;
     // universe
     uint32_t n_docs = 0;    // max docid + 1
     uint32_t n_words64 = 0; // ceil(n_docs / 64)

@@ -93,24 +93,29 @@ __device__ __forceinline__ uint32_t char_signature(const uint8_t *s, int n) {
     return m;
 }
 
-// grid.x: 256-word tiles of the dictionary; grid.y: chunks of LEV_TERMS_PER_CTA terms.
-// Two phases per group of 8 terms: (1) every thread filters its word against the 8 terms (length, first-letter rule, signature)
-// and queues the surviving (term, word) pairs in shared memory; (2) the queue is processed densely, one banded DP per thread —
-// the DP, which is the expensive part, runs on a few percent of the pairs and without divergence between matching and
-// non-matching lanes.  Match codes are collected per (term, 32-word group) and reported as ballot records.
+// One CTA per schedule item = (chunk of <= LEV_TERMS_PER_CTA terms of one group, one 256-word tile of the dictionary).
+// Words of the tile outside the group's word set (device_types.h) are skipped before any test; the rest go through the full
+// filter, first-letter rule included.  Two phases per group of 8 terms: (1) every thread filters its word against the 8 terms (length,
+// first-letter rule, signature) and queues the surviving (term, word) pairs in shared memory; (2) the queue is processed densely,
+// one banded DP per thread — the DP, which is the expensive part, runs on a few percent of the pairs and without divergence
+// between matching and non-matching lanes.  Match codes are collected per (term, 32-word group) and reported as ballot records.
 constexpr int LEV_TERM_GROUP = 8;
 __global__ void __launch_bounds__(256) lev_match_kernel(const uint8_t *__restrict__ dict_bytes, const uint32_t *__restrict__ dict_off,
-                                                        uint32_t n_words, const LevTerm *__restrict__ terms, uint32_t n_terms,
-                                                        LevRec *__restrict__ recs, uint32_t *__restrict__ rec_count) {
+                                                        uint32_t n_words, const LevTerm *__restrict__ terms,
+                                                        const uint32_t *__restrict__ term_idx, const LevChunk *__restrict__ chunks,
+                                                        const LevItem *__restrict__ items, LevRec *__restrict__ recs,
+                                                        uint32_t *__restrict__ rec_count) {
     __shared__ LevTerm sterms[LEV_TERMS_PER_CTA];
-    __shared__ uint32_t sterm_sig[LEV_TERMS_PER_CTA], sterm_meta[LEV_TERMS_PER_CTA];
+    __shared__ uint32_t sterm_sig[LEV_TERMS_PER_CTA], sterm_meta[LEV_TERMS_PER_CTA], sterm_id[LEV_TERMS_PER_CTA];
     __shared__ uint8_t sbytes[8192];
     __shared__ uint16_t s_woff[257];
     __shared__ uint32_t s_queue[LEV_TERM_GROUP * 256];  // (term << 16) | word-in-tile | (same-first << 31)
     __shared__ uint32_t s_qn;
     __shared__ unsigned long long s_codes[LEV_TERM_GROUP][8];
-    // the CTA stages its 256 dictionary words once and sweeps the term chunks blockIdx.y, blockIdx.y + gridDim.y, ... over them
-    uint32_t w0 = blockIdx.x * 256;
+    const LevItem item = items[blockIdx.x];
+    const LevChunk ch = chunks[item.chunk];
+    const uint32_t nt = ch.n;
+    uint32_t w0 = item.tile * 256;
     uint32_t wn = min(256u, n_words - w0);
     uint32_t byte0 = dict_off[w0], byte1 = dict_off[w0 + wn];
     bool in_smem = (byte1 - byte0) <= sizeof(sbytes);
@@ -118,24 +123,24 @@ __global__ void __launch_bounds__(256) lev_match_kernel(const uint8_t *__restric
         for (uint32_t i = threadIdx.x; i < byte1 - byte0; i += blockDim.x) sbytes[i] = dict_bytes[byte0 + i];
         for (uint32_t i = threadIdx.x; i <= wn; i += blockDim.x) s_woff[i] = (uint16_t)(dict_off[w0 + i] - byte0);
     }
+    if (threadIdx.x < nt) sterm_id[threadIdx.x] = term_idx[ch.first + threadIdx.x];
     __syncthreads();
+    {
+        constexpr uint32_t WORDS = sizeof(LevTerm) / 4;
+        uint32_t *dst = reinterpret_cast<uint32_t *>(sterms);
+        for (uint32_t i = threadIdx.x; i < nt * WORDS; i += blockDim.x)
+            dst[i] = reinterpret_cast<const uint32_t *>(terms + sterm_id[i / WORDS])[i % WORDS];
+    }
     uint32_t wid = w0 + threadIdx.x;
     bool valid = threadIdx.x < wn;
     uint32_t off = valid ? dict_off[wid] : byte0;
     int n = valid ? (int)(dict_off[wid + 1] - off) : 0;
     const uint8_t *w = in_smem ? (sbytes + (off - byte0)) : (dict_bytes + off);
     uint8_t w0c = n > 0 ? w[0] : 0, w1c = n > 1 ? w[1] : 0;
+    // the part of the group's word set that is the same for every term of the chunk
+    if (ch.kind == LEV_GROUP_F) valid = valid && w0c == ch.c;
+    if (ch.kind == LEV_GROUP_S) valid = valid && w1c == ch.c;
     const uint32_t wsig = char_signature(w, n);
-    const uint32_t n_chunks = (n_terms + LEV_TERMS_PER_CTA - 1) / LEV_TERMS_PER_CTA;
-    for (uint32_t chunk = blockIdx.y; chunk < n_chunks; chunk += gridDim.y) {
-    const uint32_t t0 = chunk * LEV_TERMS_PER_CTA;
-    const uint32_t nt = min((uint32_t)LEV_TERMS_PER_CTA, n_terms - t0);
-    __syncthreads();  // the previous chunk's terms are no longer read
-    {
-        const uint32_t *src = reinterpret_cast<const uint32_t *>(terms + t0);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(sterms);
-        for (uint32_t i = threadIdx.x; i < nt * sizeof(LevTerm) / 4; i += blockDim.x) dst[i] = src[i];
-    }
     __syncthreads();
     if (threadIdx.x < nt) {
         const LevTerm &T = sterms[threadIdx.x];
@@ -151,6 +156,8 @@ __global__ void __launch_bounds__(256) lev_match_kernel(const uint8_t *__restric
         // phase 1: filter, most selective test first (the signature rejects ~95 % of the pairs with two shared-memory loads)
         if (valid && n > 0) {
             for (uint32_t t = 0; t < ng; t++) {
+                // S(c): the words whose first byte is q[0] or q[1] of this term belong to its F groups
+                if (ch.kind == LEV_GROUP_S && (w0c == sterms[tg + t].q[0] || w0c == sterms[tg + t].q[1])) continue;
                 const uint32_t tsig = sterm_sig[tg + t];
                 const uint32_t meta = sterm_meta[tg + t];  // len | (k_same+1) << 8 | (k_diff+1) << 12 | prefix << 16 | q0 << 24
                 const int kmax = (int)((meta >> 8) & 15) - 1;
@@ -196,23 +203,24 @@ __global__ void __launch_bounds__(256) lev_match_kernel(const uint8_t *__restric
             }
         }
         __syncthreads();
-        // report: one record per (term, 32-word group) holding at least one match
+        // report: one record per (term, 32-word group) holding at least one match; another item of the same term may report
+        // other words of the same 32-word group (lev_finalize_kernel merges them)
         if (threadIdx.x < ng * 8) {
             const uint32_t t = threadIdx.x >> 3, g = threadIdx.x & 7;
             const unsigned long long codes = s_codes[t][g];
             if (codes) {
-                uint32_t slot = atomicAdd(&rec_count[t0 + tg + t], 1u);
+                const uint32_t term = sterm_id[tg + t];
+                uint32_t slot = atomicAdd(&rec_count[term], 1u);
                 if (slot < LEV_REC_CAP) {
                     LevRec r;
                     r.base = w0 + g * 32;
                     r.pad = 0;
                     r.codes = codes;
-                    recs[(size_t)(t0 + tg + t) * LEV_REC_CAP + slot] = r;
+                    recs[(size_t)term * LEV_REC_CAP + slot] = r;
                 }
             }
         }
         __syncthreads();
-    }
     }
 }
 
@@ -239,6 +247,15 @@ __global__ void lev_finalize_kernel(LevRec *__restrict__ recs, const uint32_t *_
         }
         r[j] = x;
     }
+    // records of one 32-word group from different items hold disjoint words: one record per group again
+    uint32_t u = 0;
+    for (uint32_t i = 0; i < cnt; i++) {
+        if (u > 0 && r[u - 1].base == r[i].base)
+            r[u - 1].codes |= r[i].codes;
+        else
+            r[u++] = r[i];
+    }
+    cnt = u;
     bool two_budget = terms[t].k_same >= 2;
     uint32_t c1 = 0, c2 = 0;
     uint32_t *o1 = one_out + (size_t)t * 150, *o2 = two_out + (size_t)t * 50;
@@ -1431,13 +1448,12 @@ cudaError_t launch_shard_merge(cudaStream_t s, const uint32_t *g_ids, const floa
     } while (0)
 
 cudaError_t launch_lev(cudaStream_t s, const uint8_t *dict_bytes, const uint32_t *dict_off, uint32_t n_words, const LevTerm *terms,
-                       uint32_t n_terms, LevRec *recs, uint32_t *rec_count, uint32_t *one_out, uint32_t *n_one, uint32_t *two_out,
-                       uint32_t *n_two, int32_t *status) {
-    if (n_terms == 0 || n_words == 0) return cudaSuccess;
+                       uint32_t n_terms, const uint32_t *term_idx, const LevChunk *chunks, const LevItem *items, uint32_t n_items,
+                       LevRec *recs, uint32_t *rec_count, uint32_t *one_out, uint32_t *n_one, uint32_t *two_out, uint32_t *n_two,
+                       int32_t *status) {
+    if (n_terms == 0) return cudaSuccess;
     CK(cudaMemsetAsync(rec_count, 0, sizeof(uint32_t) * n_terms, s));
-    const uint32_t n_chunks = (n_terms + LEV_TERMS_PER_CTA - 1) / LEV_TERMS_PER_CTA;
-    dim3 grid((n_words + 255) / 256, n_chunks < 8 ? n_chunks : 8);  // every CTA sweeps n_chunks / 8 term chunks over its word tile
-    lev_match_kernel<<<grid, 256, 0, s>>>(dict_bytes, dict_off, n_words, terms, n_terms, recs, rec_count);
+    if (n_items) lev_match_kernel<<<n_items, 256, 0, s>>>(dict_bytes, dict_off, n_words, terms, term_idx, chunks, items, recs, rec_count);
     lev_finalize_kernel<<<(n_terms + 63) / 64, 64, 0, s>>>(recs, rec_count, terms, n_terms, one_out, n_one, two_out, n_two, status);
     return cudaGetLastError();
 }

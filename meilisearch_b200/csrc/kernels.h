@@ -5,9 +5,11 @@
 #include "device_types.h"
 
 namespace b200 {
+// items / chunks / term_idx: the pruned schedule of Engine::derive_batch (one CTA per item)
 cudaError_t launch_lev(cudaStream_t s, const uint8_t *dict_bytes, const uint32_t *dict_off, uint32_t n_words, const LevTerm *terms,
-                       uint32_t n_terms, LevRec *recs, uint32_t *rec_count, uint32_t *one_out, uint32_t *n_one, uint32_t *two_out,
-                       uint32_t *n_two, int32_t *status);
+                       uint32_t n_terms, const uint32_t *term_idx, const LevChunk *chunks, const LevItem *items, uint32_t n_items,
+                       LevRec *recs, uint32_t *rec_count, uint32_t *one_out, uint32_t *n_one, uint32_t *two_out, uint32_t *n_two,
+                       int32_t *status);
 // tiles: one per COMPACT_SEG parent rows of every activation; seg_count: n_tiles u32 scratch; multi_segment: some activation has > 1 segment
 cudaError_t launch_compact(cudaStream_t s, const CompactTile *tiles, uint32_t n_tiles, bool multi_segment, const ActDesc *acts,
                            uint32_t *seg_count, uint32_t *results);
